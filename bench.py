@@ -85,7 +85,16 @@ def parse():
     ap.add_argument("--sm-caps", default="",
                     help="pipelined step: persistent-grid caps 'fwd:bwd' of sa1,sa2,sa3,sa4,vote-agg "
                          "(comma separated, 0 = every SM); default: see PipelinedTrainStep")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="after the timed steps, run ONE EXTRA, untimed step of the timed path (same captured "
+                         "graph) from the initial weights on the first batch, and write what it produced to "
+                         "DIR/<name>.npy (float32): the loss, the gradient of every parameter and the BatchNorm "
+                         "running statistics.  Not the last timed step: the timed trajectory does not repeat "
+                         "bit for bit (atomics in the fused backward, carried on by Adam)")
     a = ap.parse_args()
+    if a.dump_outputs and os.environ.get("B2R_PINGPONG", "0") not in ("0", ""):
+        # two captured graphs alternate; the gradient tensors of only one of them are kept
+        ap.error("--dump-outputs is not supported with B2R_PINGPONG=1")
     if a.batch <= 0:
         a.batch = 4 if a.workload == "gf3d" else 8
     if a.npoints <= 0:
@@ -295,7 +304,8 @@ def reference_gpu_steps(a, dev, steps=10, warmup=3):
 def run_leg(a):
     """Internal (--leg): one of the product arm's reference legs, in its own process."""
     if a.leg == "reference_gpu":
-        res = reference_gpu_steps(a, torch.device("cuda", 0)) if torch.cuda.is_available() else None
+        res = (reference_gpu_steps(a, torch.device("cuda", 0), a.steps, a.warmup)
+               if torch.cuda.is_available() else None)
         emit(res or {})
     else:
         per = scenes_per_step(a) if a.cpu_scenes >= a.batch else (
@@ -452,6 +462,27 @@ def trace_steps(path, fn, steps=3):
         print("timeline dump failed: %r" % (e,), file=sys.stderr)
 
 
+def dump_outputs(out_dir, loss, net, grads):
+    """What the training step hands its caller: the loss, the gradients (parameter order) and the
+    BatchNorm running statistics.  The updated parameters are left out: Adam normalises its update
+    per element, which turns rounding noise in a near-zero gradient into a step of up to lr."""
+    torch.cuda.synchronize()
+    arrays = {"loss": loss}
+    for (name, _), g in zip(net.named_parameters(), grads):
+        if g is not None:
+            arrays["grad." + name] = g
+    for name, b in net.named_buffers():
+        if b.is_floating_point():
+            arrays["buffer." + name] = b
+    arrays = {k: v.detach().float().cpu().numpy() for k, v in arrays.items()}
+    total = sum(v.nbytes for v in arrays.values())
+    assert total <= 64 << 20, "outputs of %d bytes exceed the 64 MB dump limit" % total
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), v)
+    log("wrote %d arrays (%.1f MB) to %s" % (len(arrays), total / 2**20, out_dir))
+
+
 # ------------------------------------------------------------------------- GPU arm ---------
 def run_b2r(a):
     import torch.distributed as dist
@@ -507,6 +538,9 @@ def run_b2r(a):
         bucket = dist_utils.FlatGradBucket(params, as_views=False) if world > 1 else None
         opt = torch.optim.Adam(params, lr=1e-3, fused=True, capturable=True)
     live = {"grads": None}   # the gradient tensors the last backward (or the graph) produced
+    # --dump-outputs: the weights and BatchNorm statistics the dumped step starts from
+    initial = ([t.detach().clone() for t in list(net.parameters()) + list(net.buffers())]
+               if a.dump_outputs else None)
 
     pool_n = 4
     host = [torch.from_numpy(make_batch(a, rank * pool_n + i)).pin_memory() for i in range(pool_n)]
@@ -699,6 +733,19 @@ def run_b2r(a):
         clocks = sampler.window(t0, t1e)
         sampler.stop()
 
+    if a.dump_outputs:
+        # One more step of the same path after the timed ones, from the initial weights and on a
+        # fixed batch.  The timed trajectory does not repeat bit for bit (the fused backward sums
+        # with atomics) and Adam carries that noise on from step to step; one step from a fixed
+        # state repeats to within rounding, so two builds compare array by array.
+        with torch.no_grad():
+            for t, v in zip(list(net.parameters()) + list(net.buffers()), initial):
+                t.copy_(v)
+        prime()
+        loss = run_step(resident[nxt % pool_n])
+        if rank == 0:
+            dump_outputs(a.dump_outputs, loss, net, live["grads"])
+
     if a.trace and rank == 0:
         trace_steps(a.trace, lambda i: run_step(resident[(i + nxt) % pool_n]))
 
@@ -809,6 +856,8 @@ def run_b2r(a):
             try:
                 cmd = [sys.executable, os.path.abspath(__file__), "--leg", leg, "--workload", a.workload,
                        "--batch", str(a.batch), "--npoints", str(a.npoints), "--cpu-scenes", str(a.cpu_scenes)]
+                if leg == "reference_gpu":    # the CPU leg times a fixed 3-step sample (see run_leg)
+                    cmd += ["--steps", str(a.steps), "--warmup", str(a.warmup)]
                 r = subprocess.run(cmd, capture_output=True, text=True, timeout=900)
                 line = [ln for ln in r.stdout.splitlines() if ln.startswith("{")]
                 if line:
@@ -825,7 +874,8 @@ def run_b2r(a):
         log("timing leg unfused_tf32 in a subprocess ...")
         try:
             cmd = [sys.executable, os.path.abspath(__file__), "--workload", a.workload, "--batch", str(a.batch),
-                   "--npoints", str(a.npoints), "--steps", "10", "--warmup", "3", "--no-cpu-baseline"]
+                   "--npoints", str(a.npoints), "--steps", str(a.steps), "--warmup", str(a.warmup),
+                   "--no-cpu-baseline"]
             env = dict(os.environ, B2R_FUSED="0", B2R_DENSE="0")
             r = subprocess.run(cmd, capture_output=True, text=True, timeout=600, env=env)
             line = [ln for ln in r.stdout.splitlines() if ln.startswith("{")]

@@ -1,4 +1,4 @@
-"""Checks that need the reference tree (/root/reference): skipped on the GPU box.
+"""Checks that need the reference tree (oracle/ref_python.py: B2R_REFERENCE_ROOT); skipped without it.
 
 * the reference's ONLY test, pointnet2_test.py:18-30 (gradcheck of three_interpolate), run
   verbatim in spirit on CPU over the oracle `_ext` (double perturbation is applied by gradcheck
@@ -73,7 +73,7 @@ def test_nn_distance_oracle_equals_reference_module_on_cpu():
 
     import pytest
     import torch
-    path = "/root/reference/detection/Votenet/utils/nn_distance.py"
+    path = os.path.join(ref_python.REF_ROOT, "detection", "Votenet", "utils", "nn_distance.py")
     if not os.path.isfile(path):
         pytest.skip("reference tree not present")
     spec = importlib.util.spec_from_file_location("ref_nn_distance", path)
