@@ -160,6 +160,32 @@ SIGNATURES.update({
 })
 _RESTYPES["b2r_dense_image_bytes"] = ctypes.c_longlong
 
+
+ADAM_MAX_GROUPS = 64    # B2R_ADAM_MAX_GROUPS
+
+
+class AdamGroup(ctypes.Structure):
+    """struct b2r_adam_group (include/b2r.h): one entry of the device table."""
+    _fields_ = [("start", _ll), ("end", _ll), ("lr", _f), ("weight_decay", _f)]
+
+
+class AdamDesc(ctypes.Structure):
+    """struct b2r_adam_desc (include/b2r.h)."""
+    _fields_ = [
+        ("params", _vp), ("grads", _vp), ("exp_avg", _vp), ("exp_avg_sq", _vp), ("n", _ll),
+        ("state", _vp), ("groups", _vp), ("n_groups", _i),
+        ("beta1", _f), ("beta2", _f), ("eps", _f), ("grad_scale", _f), ("decoupled", _i),
+        ("clip_coef", _vp),
+    ]
+
+
+SIGNATURES.update({
+    "b2r_adam_flat_step_groups": [ctypes.POINTER(AdamDesc), _vp],
+    "b2r_flat_grad_norm_workspace_bytes": [_ll],
+    "b2r_flat_grad_norm": [_vp, _ll, _f, _f, _vp, _vp, _vp, _vp],
+})
+_RESTYPES["b2r_flat_grad_norm_workspace_bytes"] = ctypes.c_longlong
+
 _lib = None
 
 

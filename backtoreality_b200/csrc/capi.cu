@@ -36,6 +36,7 @@ extern "C" int b2r_struct_bytes(int which) {
   if (which == 1) return (int)sizeof(b2r_sa_layer_bwd_desc);
   if (which == 2) return (int)sizeof(b2r_dense_layer);
   if (which == 3) return (int)sizeof(b2r_dense_layer_bwd);
+  if (which == 4) return (int)sizeof(b2r_adam_desc);
   return -1;
 }
 

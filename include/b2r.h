@@ -47,7 +47,7 @@ B2R_API int b2r_version(void);
 B2R_API const char *b2r_status_string(int status);
 B2R_API const char *b2r_last_error(void);
 /* sizeof() of the descriptor structs as THIS build of the library sees them (0: b2r_sa_layer,
- * 1: b2r_sa_layer_bwd_desc, 2: b2r_dense_layer, 3: b2r_dense_layer_bwd; -1 otherwise): lets a binding in another language verify its mirror
+ * 1: b2r_sa_layer_bwd_desc, 2: b2r_dense_layer, 3: b2r_dense_layer_bwd, 4: b2r_adam_desc; -1 otherwise): lets a binding in another language verify its mirror
  * of the struct layout before the first launch (tests/test_capi_symbols.py does). */
 B2R_API int b2r_struct_bytes(int which);
 
@@ -498,6 +498,50 @@ B2R_API int b2r_adam_state_bytes(void);
 B2R_API int b2r_adam_flat_step(float *params, const float *grads, float *exp_avg, float *exp_avg_sq,
                                long long n, void *state, float lr, float beta1, float beta2, float eps,
                                float weight_decay, float grad_scale, void *stream);
+
+/* Parameter groups (torch.optim param_groups) of the flat buffer: elements [start, end) with their
+ * own learning rate and weight decay.  The table lives in DEVICE memory and is read by every
+ * launch, so rates written into it between CUDA-graph replays (a learning-rate schedule) apply to
+ * the next replay.  Entries are sorted and disjoint; start is a multiple of 4 and end is a multiple
+ * of 4 or n, so that every 16-byte vector of the buffer lies in one group.  Elements outside every
+ * group are left untouched. */
+#define B2R_ADAM_MAX_GROUPS 64
+typedef struct b2r_adam_group {
+  long long start, end;
+  float lr, weight_decay;
+} b2r_adam_group;
+
+/* One Adam / AdamW step over parameter groups (b2r_struct_bytes(4) is sizeof this struct).
+ * Buffers as for b2r_adam_flat_step (n floats each, 16-byte aligned; state: the step counter).
+ * decoupled = 0: torch.optim.Adam's L2 decay g += wd*p; 1: torch.optim.AdamW's p *= 1 - lr*wd
+ * before the moment update.  The gradient is multiplied by grad_scale and then, when clip_coef is
+ * not NULL, by the device scalar *clip_coef (b2r_flat_grad_norm's coef_out). */
+typedef struct b2r_adam_desc {
+  float *params;
+  const float *grads;
+  float *exp_avg, *exp_avg_sq;
+  long long n;
+  void *state;
+  const b2r_adam_group *groups; /* device table, n_groups entries (1..B2R_ADAM_MAX_GROUPS) */
+  int n_groups;
+  float beta1, beta2, eps;
+  float grad_scale;
+  int decoupled;
+  const float *clip_coef; /* device scalar or NULL */
+} b2r_adam_desc;
+B2R_API int b2r_adam_flat_step_groups(const b2r_adam_desc *desc, void *stream);
+
+/* Global L2 norm of grad_scale * grads (n floats, 16-byte aligned) -- torch.nn.utils.
+ * clip_grad_norm_(..., max_norm, norm_type=2) without modifying the gradients.  Writes the norm to
+ * the device scalar *norm_out and min(max_norm / (norm + 1e-6), 1) to *coef_out (fp32, torch's
+ * clip_coef_clamped: a NaN norm gives NaN, an infinite one 0).  Two launches: a fixed grid (its
+ * size depends on n only) of fp64 partial sums of squares, then one block that adds the partials
+ * in a fixed order.  No atomics: identical gradients give a bit-identical norm.  No host
+ * synchronisation: graph-capturable.  workspace: b2r_flat_grad_norm_workspace_bytes(n) bytes of
+ * device memory, 16-byte aligned (-1 for n < 0). */
+B2R_API long long b2r_flat_grad_norm_workspace_bytes(long long n);
+B2R_API int b2r_flat_grad_norm(const float *grads, long long n, float grad_scale, float max_norm,
+                               void *workspace, float *norm_out, float *coef_out, void *stream);
 
 #ifdef __cplusplus
 }
