@@ -724,6 +724,8 @@ extern "C" int b2r_bn_finalize(const double *stats, int C, double count, const f
                                float *running_var, float *scale, float *shift, float *mean_out,
                                float *invstd_out, long long *num_batches_tracked, void *stream) {
   B2R_REQUIRE(stats && scale && shift && C > 0 && count > 0, "b2r_bn_finalize: bad argument");
+  B2R_REQUIRE((running_mean == nullptr) == (running_var == nullptr),
+              "b2r_bn_finalize: running_mean and running_var must both be given or both be NULL");
   bn_finalize_kernel<<<ceil_div(C, 128), 128, 0, static_cast<cudaStream_t>(stream)>>>(
       stats, C, 1.0 / count, count > 1.0 ? (float)(count / (count - 1.0)) : 1.0f, gamma, beta, eps,
       momentum, running_mean, running_var, scale, shift,

@@ -275,7 +275,8 @@ B2R_API int b2r_sa_layer_fwd_tile(int B, int NP, int NS, int Cin, int Cout, int 
 /* BatchNorm bookkeeping from accumulated statistics (replaces the statistics half of
  * nn.BatchNorm2d in training mode, reference pytorch_utils.py:55-58): scale = gamma*invstd,
  * shift = beta - mean*scale; running stats updated with `momentum` (unbiased variance) when
- * running_mean/var are non-NULL; *num_batches_tracked (int64, may be NULL) is incremented.
+ * running_mean/var are non-NULL (both or neither, else B2R_ERR_INVALID_ARG);
+ * *num_batches_tracked (int64, may be NULL) is incremented.
  * mean_out / invstd_out (C) are optional (saved for backward). */
 B2R_API int b2r_bn_finalize(const double *stats, int C, double count, const float *gamma,
                             const float *beta, float eps, float momentum, float *running_mean,

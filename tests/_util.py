@@ -50,10 +50,11 @@ def round_bf16(t):
     return t.detach().float().bfloat16().float()
 
 
-def emu_log(name, **errs):
+def emu_log(name, log="emulation_parity.log", **errs):
     """Tests that compare a kernel with its operand-rounding emulation record the measured error
-    (gpurun_out/emulation_parity.log when that directory exists) so the bounds can be audited."""
+    (file `log` in the run's output directory, when that directory exists) so the bounds can be
+    audited."""
     d = os.path.join(os.path.dirname(GOLDEN[:-len("/golden")]), "gpurun_out")
     if os.path.isdir(d):
-        with open(os.path.join(d, "emulation_parity.log"), "a") as f:
+        with open(os.path.join(d, log), "a") as f:
             f.write(name + "  " + "  ".join("%s %.2e" % kv for kv in errs.items()) + "\n")
