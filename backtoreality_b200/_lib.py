@@ -78,6 +78,8 @@ SIGNATURES.update({
     "b2r_sa_layer_fwd_supported": [_i, _i, _i, _i, _i, _i, _i],
     "b2r_bn_finalize": [_vp, _i, ctypes.c_double, _vp, _vp, _f, _f, _vp, _vp, _vp, _vp, _vp, _vp,
                         _vp, _vp],
+    "b2r_bn_finalize_dev": [_vp, _i, ctypes.c_double, _vp, _vp, _f, _vp, _vp, _vp, _vp, _vp, _vp,
+                            _vp, _vp, _vp],
     "b2r_pool_finalize": [_vp, _vp, _vp, _vp, _i, _i, _i, _vp, _vp, _vp],
     "b2r_to_point_major": [_vp, _i, _i, _i, _vp, _vp],
 })

@@ -474,10 +474,15 @@ __global__ void __launch_bounds__(kFwdThreads, 1) sa_layer_fwd_kernel(const Laye
 // BatchNorm bookkeeping from the accumulated statistics (one thread per channel):
 //   scale = gamma / sqrt(var_biased + eps), shift = beta - mean * scale        (training)
 //   running_mean/var updated with `momentum` (unbiased variance), like nn.BatchNorm2d
+// kDevMomentum: the momentum is read from device memory (*momentum_dev) when the kernel runs, so a
+// replayed CUDA graph follows a momentum schedule; otherwise it is the by-value `momentum`.
+template <bool kDevMomentum>
 __global__ void bn_finalize_kernel(const double *__restrict__ stats, int Cch, double inv_count,
                                    float unbias,
                                    const float *__restrict__ gamma, const float *__restrict__ beta,
-                                   float eps, float momentum, float *__restrict__ running_mean,
+                                   float eps, float momentum_val,
+                                   const float *__restrict__ momentum_dev,
+                                   float *__restrict__ running_mean,
                                    float *__restrict__ running_var, float *__restrict__ scale,
                                    float *__restrict__ shift, float *__restrict__ mean_out,
                                    float *__restrict__ invstd_out,
@@ -499,6 +504,7 @@ __global__ void bn_finalize_kernel(const double *__restrict__ stats, int Cch, do
   if (mean_out) mean_out[ch] = (float)mean;
   if (invstd_out) invstd_out[ch] = invstd;
   if (running_mean) {
+    const float momentum = kDevMomentum ? *momentum_dev : momentum_val;
     const float unbiased = (float)var * unbias;
     running_mean[ch] = (1.f - momentum) * running_mean[ch] + momentum * (float)mean;
     running_var[ch] = (1.f - momentum) * running_var[ch] + momentum * unbiased;
@@ -719,19 +725,43 @@ extern "C" int b2r_sa_layer_fwd(const b2r_sa_layer *d, void *stream) {
   return B2R_OK;
 }
 
+// the two entries below: same validation, same kernel template, momentum by value or on the device
+template <bool kDevMomentum>
+static int bn_finalize_launch(const char *name, const double *stats, int C, double count,
+                              const float *gamma, const float *beta, float eps, float momentum,
+                              const float *momentum_dev, float *running_mean, float *running_var,
+                              float *scale, float *shift, float *mean_out, float *invstd_out,
+                              long long *num_batches_tracked, void *stream) {
+  B2R_REQUIRE(stats && scale && shift && C > 0 && count > 0, "%s: bad argument", name);
+  B2R_REQUIRE((running_mean == nullptr) == (running_var == nullptr),
+              "%s: running_mean and running_var must both be given or both be NULL", name);
+  B2R_REQUIRE(!kDevMomentum || running_mean == nullptr || momentum_dev != nullptr,
+              "%s: running statistics given without a momentum pointer", name);
+  bn_finalize_kernel<kDevMomentum><<<ceil_div(C, 128), 128, 0, static_cast<cudaStream_t>(stream)>>>(
+      stats, C, 1.0 / count, count > 1.0 ? (float)(count / (count - 1.0)) : 1.0f, gamma, beta, eps,
+      momentum, momentum_dev, running_mean, running_var, scale, shift,
+      mean_out, invstd_out, num_batches_tracked);
+  B2R_CHECK_LAUNCH();
+  return B2R_OK;
+}
+
 extern "C" int b2r_bn_finalize(const double *stats, int C, double count, const float *gamma,
                                const float *beta, float eps, float momentum, float *running_mean,
                                float *running_var, float *scale, float *shift, float *mean_out,
                                float *invstd_out, long long *num_batches_tracked, void *stream) {
-  B2R_REQUIRE(stats && scale && shift && C > 0 && count > 0, "b2r_bn_finalize: bad argument");
-  B2R_REQUIRE((running_mean == nullptr) == (running_var == nullptr),
-              "b2r_bn_finalize: running_mean and running_var must both be given or both be NULL");
-  bn_finalize_kernel<<<ceil_div(C, 128), 128, 0, static_cast<cudaStream_t>(stream)>>>(
-      stats, C, 1.0 / count, count > 1.0 ? (float)(count / (count - 1.0)) : 1.0f, gamma, beta, eps,
-      momentum, running_mean, running_var, scale, shift,
-      mean_out, invstd_out, num_batches_tracked);
-  B2R_CHECK_LAUNCH();
-  return B2R_OK;
+  return bn_finalize_launch<false>("b2r_bn_finalize", stats, C, count, gamma, beta, eps, momentum,
+                                   nullptr, running_mean, running_var, scale, shift, mean_out,
+                                   invstd_out, num_batches_tracked, stream);
+}
+
+extern "C" int b2r_bn_finalize_dev(const double *stats, int C, double count, const float *gamma,
+                                   const float *beta, float eps, const float *momentum,
+                                   float *running_mean, float *running_var, float *scale,
+                                   float *shift, float *mean_out, float *invstd_out,
+                                   long long *num_batches_tracked, void *stream) {
+  return bn_finalize_launch<true>("b2r_bn_finalize_dev", stats, C, count, gamma, beta, eps, 0.f,
+                                  momentum, running_mean, running_var, scale, shift, mean_out,
+                                  invstd_out, num_batches_tracked, stream);
 }
 
 extern "C" int b2r_pool_finalize(const float *zmax, const float *zmin, const float *scale,

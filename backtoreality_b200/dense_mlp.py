@@ -24,7 +24,7 @@ import os
 
 import torch
 
-from . import _ext, _lib, step_arena
+from . import _ext, _lib, pytorch_utils, step_arena
 
 _vp = ctypes.c_void_p
 
@@ -205,11 +205,7 @@ class _DenseMLP(torch.autograd.Function):
                 if training:
                     mean = torch.empty(Cout, dtype=torch.float32, device=dev)
                     invstd = torch.empty_like(mean)
-                    _lib.check(lib.b2r_bn_finalize(
-                        _ptr(stats), Cout, float(M), _ptr(bn.weight), _ptr(bn.bias), float(bn.eps),
-                        float(bn.momentum), _ptr(bn.running_mean), _ptr(bn.running_var), _ptr(sc),
-                        _ptr(sh), _ptr(mean), _ptr(invstd), _ptr(bn.num_batches_tracked), st),
-                        "bn_finalize")
+                    pytorch_utils.bn_finalize(bn, stats, Cout, M, sc, sh, mean, invstd, st)
                     _ext.LAUNCHES += 1
                 else:
                     invstd = torch.rsqrt(bn.running_var + bn.eps)

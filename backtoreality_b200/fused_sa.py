@@ -34,7 +34,7 @@ import os
 
 import torch
 
-from . import _ext, _lib, step_arena
+from . import _ext, _lib, pytorch_utils, step_arena
 
 _vp = ctypes.c_void_p
 
@@ -291,12 +291,7 @@ def sa_mlp_forward(xyz, new_xyz, feat_t, idx, radius, normalize_xyz, mlp_module,
             shift = torch.empty_like(scale)
             mean = torch.empty_like(scale)
             invstd = torch.empty_like(scale)
-            _lib.check(lib.b2r_bn_finalize(_ptr(stats), Cout, float(M), _ptr(bn.weight),
-                                           _ptr(bn.bias), float(bn.eps), float(bn.momentum),
-                                           _ptr(bn.running_mean), _ptr(bn.running_var),
-                                           _ptr(scale), _ptr(shift), _ptr(mean), _ptr(invstd),
-                                           _ptr(bn.num_batches_tracked), st),
-                       "bn_finalize")
+            pytorch_utils.bn_finalize(bn, stats, Cout, M, scale, shift, mean, invstd, st)
             _ext.LAUNCHES += 1
         else:
             invstd = torch.rsqrt(bn.running_var + bn.eps)

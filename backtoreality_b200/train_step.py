@@ -7,16 +7,19 @@ reads), so forward + backward + gradient all-reduce + optimizer are captured ONC
 graph and replayed: one launch per step, no gaps.
 
 Values that are baked in at capture time: tensor addresses (the input is a static buffer that
-`__call__` copies into), BatchNorm momentum (a Python float the reference's BNMomentumScheduler
-changes once per epoch, pytorch_utils.py:262-296 -> call `recapture()` after changing it) and the
-learning rate unless it is a tensor.
+`__call__` copies into) and the learning rate unless the optimizer reads it from the device
+(flat_adam.FlatAdam.sync_hparams).  The BatchNorm momentum, which the reference's
+BNMomentumScheduler changes once per epoch (pytorch_utils.py:262-296), replays from a device table
+once `pytorch_utils.sync_bn_momentum(model)` has attached the model before the capture;
+BNMomentumScheduler.step() then updates that table between replays.  A model that is not
+attached keeps its capture-time momentum until `recapture()`.
 
 The warm-up steps that precede a capture are REAL steps on the static batch.  Pass
 `snapshot=[model, optimizer, ...]` (anything with state_dict / load_state_dict) and their state
 -- weights, BatchNorm running statistics and num_batches_tracked, optimizer moments and step
 counts -- is saved before the warm-up and restored after it, so a (re)capture leaves training
-exactly where it was (a recapture per epoch, after BNMomentumScheduler.step(), would otherwise
-add `warmup` weight updates on duplicated data each time).
+exactly where it was (each recapture would otherwise add `warmup` weight updates on duplicated
+data).
 """
 import copy
 
@@ -108,7 +111,8 @@ class PipelinedTrainStep:
     Pointnet2Backbone.forward), backward and the optimizer.  Every call does one geometry pre-pass
     and one full step, so K calls cost K of each: nothing is skipped, only re-ordered.
     `__call__(next_batch)` returns the loss of the batch submitted by the PREVIOUS call (or by
-    the constructor / `prime`).  BatchNorm momentum / learning-rate caveats as CapturedTrainStep.
+    the constructor / `prime`).  What is baked in at capture, and what replays from the device
+(learning rate, BatchNorm momentum), as for CapturedTrainStep.
     """
 
     GEO_KEYS = ("inds", "new_xyz", "idx")                       # every level

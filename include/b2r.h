@@ -283,6 +283,15 @@ B2R_API int b2r_bn_finalize(const double *stats, int C, double count, const floa
                             float *running_var, float *scale, float *shift, float *mean_out,
                             float *invstd_out, long long *num_batches_tracked, void *stream);
 
+/* b2r_bn_finalize with the momentum in device memory (one float), read when the kernel runs: a
+ * captured CUDA graph then follows a momentum written between replays.  Same validation, plus
+ * B2R_ERR_INVALID_ARG when running_mean/var are given and `momentum` is NULL. */
+B2R_API int b2r_bn_finalize_dev(const double *stats, int C, double count, const float *gamma,
+                                const float *beta, float eps, const float *momentum,
+                                float *running_mean, float *running_var, float *scale,
+                                float *shift, float *mean_out, float *invstd_out,
+                                long long *num_batches_tracked, void *stream);
+
 /* out = relu(scale*(scale>=0 ? zmax : zmin) + shift): (B,C,NP) channel-major (reference layout)
  * and/or (B,NP,C) point-major (the next layer's gather source).  Either output may be NULL. */
 B2R_API int b2r_pool_finalize(const float *zmax, const float *zmin, const float *scale,
