@@ -68,14 +68,17 @@ class SaLayer(ctypes.Structure):
         ("zmax", _vp), ("zmin", _vp), ("amax", _vp), ("amin", _vp),
         ("sm_limit", _i),
         ("cidx", _vp), ("ccen", _vp), ("cmeta", _vp),
+        ("co0", _i), ("co_n", _i), ("ci0", _i), ("ci_n", _i), ("accumulate", _i),
     ]
 
 
+_ip = ctypes.POINTER(_i)
 SIGNATURES.update({
     "b2r_mlp_weight_image_bytes": [_i, _i, _i],
     "b2r_mlp_pack_weight": [_vp, _i, _i, _i, _vp, _vp],
     "b2r_sa_layer_fwd": [ctypes.POINTER(SaLayer), _vp],
     "b2r_sa_layer_fwd_supported": [_i, _i, _i, _i, _i, _i, _i],
+    "b2r_sa_layer_fwd_slices": [_i, _i, _i, _i, _ip, _ip],
     "b2r_bn_finalize": [_vp, _i, ctypes.c_double, _vp, _vp, _f, _f, _vp, _vp, _vp, _vp, _vp, _vp,
                         _vp, _vp],
     "b2r_bn_finalize_dev": [_vp, _i, ctypes.c_double, _vp, _vp, _f, _vp, _vp, _vp, _vp, _vp, _vp,
@@ -100,6 +103,7 @@ class SaLayerBwd(ctypes.Structure):
         ("g_feat_t", _vp), ("g_xyz", _vp), ("g_new_xyz", _vp),
         ("sm_limit", _i),
         ("cidx", _vp), ("ccen", _vp), ("cmeta", _vp),
+        ("co0", _i), ("co_n", _i), ("ci0", _i), ("ci_n", _i), ("accumulate", _i),
     ]
 
 
@@ -108,6 +112,7 @@ SIGNATURES.update({
     "b2r_mlp_pack_weight_bf16": [_vp, _i, _i, _i, _vp, _vp],
     "b2r_sa_layer_bwd": [ctypes.POINTER(SaLayerBwd), _vp],
     "b2r_sa_layer_bwd_supported": [_i, _i, _i, _i, _i, _i, _i],
+    "b2r_sa_layer_bwd_slices": [_i, _i, _i, _i, _ip, _ip],
     "b2r_pool_bwd_prep": [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _vp, _vp, _vp, _vp],
     "b2r_bn_bwd_finalize": [_vp, _i, ctypes.c_double, _vp, _vp, _vp, _i, _vp, _vp, _vp, _vp, _vp,
                             _vp, _vp, _vp, _vp],

@@ -25,29 +25,31 @@ _QUERY_STREAMS = {}  # (device, side stream) -> second side stream (ball queries
 
 class Pointnet2Backbone(nn.Module):
     """input_feature_dim: channels per point beyond xyz (1 = height for VoteNet, 0 for GF3D).
-    fp2_out: 256 (VoteNet) or 288 (GroupFree3D).  width / depth: accepted for signature parity
-    with the GroupFree3D reference (models/backbone_module.py:21-33), whose constructor takes
-    them; only the published configuration width = 1, depth = 2 is built (it fixes the SA / FP
-    channel tables above and the state-dict layout)."""
+    fp2_out: 256 (VoteNet) or 288 (GroupFree3D).  width / depth: the GroupFree3D reference's
+    channel multiplier and number of hidden layers per SA block (models/backbone_module.py:21-33);
+    width=1, depth=2 is the published default and VoteNet's backbone, width=2 the "w2x" models.
+    Layers too wide for one fused launch run as channel-slice launches (fused_sa.slice_grid)."""
 
     def __init__(self, input_feature_dim=0, fp2_out=256, width=1, depth=2):
         super().__init__()
-        if width != 1 or depth != 2:
-            raise NotImplementedError("only width=1, depth=2 (the reference's defaults) are built")
+        if int(width) != width or width < 1 or int(depth) != depth or depth < 1:
+            raise ValueError("width and depth must be integers >= 1 (got %r, %r)" % (width, depth))
+        w, d = int(width), int(depth)
+        self.width, self.depth = w, d
         self.sa1 = PointnetSAModuleVotes(npoint=2048, radius=0.2, nsample=64,
-                                         mlp=[input_feature_dim, 64, 64, 128],
+                                         mlp=[input_feature_dim] + [64 * w] * d + [128 * w],
                                          use_xyz=True, normalize_xyz=True)
         self.sa2 = PointnetSAModuleVotes(npoint=1024, radius=0.4, nsample=32,
-                                         mlp=[128, 128, 128, 256],
+                                         mlp=[128 * w] + [128 * w] * d + [256 * w],
                                          use_xyz=True, normalize_xyz=True)
         self.sa3 = PointnetSAModuleVotes(npoint=512, radius=0.8, nsample=16,
-                                         mlp=[256, 128, 128, 256],
+                                         mlp=[256 * w] + [128 * w] * d + [256 * w],
                                          use_xyz=True, normalize_xyz=True)
         self.sa4 = PointnetSAModuleVotes(npoint=256, radius=1.2, nsample=16,
-                                         mlp=[256, 128, 128, 256],
+                                         mlp=[256 * w] + [128 * w] * d + [256 * w],
                                          use_xyz=True, normalize_xyz=True)
-        self.fp1 = PointnetFPModule(mlp=[256 + 256, 256, 256])
-        self.fp2 = PointnetFPModule(mlp=[256 + 256, 256, fp2_out])
+        self.fp1 = PointnetFPModule(mlp=[512 * w, 256 * w, 256 * w])
+        self.fp2 = PointnetFPModule(mlp=[512 * w, 256 * w, fp2_out])
 
     def _break_up_pc(self, pc):
         xyz = pc[..., 0:3].contiguous()

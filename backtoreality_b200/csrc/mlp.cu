@@ -28,6 +28,10 @@
 // with tcgen05.ld.32x32b.x32, MMA completion signalled through tcgen05.commit -> mbarrier.
 // The weight operand is staged by the TMA unit: one cp.async.bulk (UBLKCP) of a pre-swizzled
 // weight image built by `pack_weight_kernel`.
+// A layer whose image does not fit (or with Cout > 256) runs as a grid of channel-slice launches
+// of the same kernel (b2r_sa_layer_fwd_slices, DESIGN.md section 4): output slices write their own
+// columns of the whole layer's z / statistics / pool outputs; feature slices of a gather layer add
+// their partial z in the storing epilogue (ldz, ldf, accumulate in LayerArgs).
 #include "mlp_common.cuh"
 
 namespace b2r {
@@ -74,6 +78,10 @@ struct LayerArgs {
   int *amax, *amin;
   int Kp, Cout_pad, num_tiles, chf_shift, ns_shift, raw_stage;
   const int *cidx, *ccen, *cmeta;   // compacted position space (csrc/compact.cu) or NULL
+  // channel slice: row pitch of z / zmax / zmin / amax / amin and offset of the sum-of-squares
+  // half of stats (the whole layer's Cout; Cout above is the slice's), row pitch of feat_t, and
+  // z += product instead of z = product (a feature slice after the first)
+  int ldz, ldf, accumulate;
 };
 
 // Warp roles (16 warps = 4 per SM sub-partition -> 128 registers/thread):
@@ -133,7 +141,9 @@ __device__ __forceinline__ void mbar_arrive1(uint32_t bar) {
 // the plan's meta words on the device, gather rows from cidx / ccen, and the epilogue works on
 // 8-column sample groups whose class (8/16/32/64 samples per centre), liveness and first-sample
 // weight are per-TILE constants.
-template <int NT, bool CMP>
+// SL: a channel-slice launch (ldz / ldf / accumulate); the whole-layer instantiations keep the
+// arithmetic and addressing they had before slices existed
+template <int NT, bool CMP, bool SL>
 __global__ void __launch_bounds__(kFwdThreads, 1) sa_layer_fwd_kernel(const LayerArgs a) {
   extern __shared__ __align__(1024) uint8_t smem_raw[];
   uint8_t *base = reinterpret_cast<uint8_t *>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) &
@@ -153,6 +163,7 @@ __global__ void __launch_bounds__(kFwdThreads, 1) sa_layer_fwd_kernel(const Laye
 
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const int MT = a.Cout_pad >> 7;
+  const int ldz = SL ? a.ldz : a.Cout;
   constexpr int NCH = NT / 32;
   constexpr uint32_t kTmemCols = 512;
   const int grid = (int)gridDim.x;
@@ -192,7 +203,7 @@ __global__ void __launch_bounds__(kFwdThreads, 1) sa_layer_fwd_kernel(const Laye
     gsrc.xyz = a.xyz; gsrc.new_xyz = a.new_xyz; gsrc.feat_t = a.feat_t;
     gsrc.N = a.N; gsrc.NP = a.NP; gsrc.NS = a.NS; gsrc.C = a.Cin - 3;
     gsrc.Cf4 = (a.Cin - 3 + 3) & ~3;
-    gsrc.chf_shift = a.chf_shift; gsrc.radius = a.radius; gsrc.normalize_xyz = a.normalize_xyz;
+    gsrc.ldf = SL ? a.ldf : gsrc.C; gsrc.chf_shift = a.chf_shift; gsrc.radius = a.radius; gsrc.normalize_xyz = a.normalize_xyz;
     if (a.raw_stage && ptid == 0) {   // prime the raw ring with this CTA's first two tiles
       for (int k = 0; k < 2; ++k) {
         const long long tile = (long long)blockIdx.x + (long long)k * grid;
@@ -375,13 +386,20 @@ __global__ void __launch_bounds__(kFwdThreads, 1) sa_layer_fwd_kernel(const Laye
         const uint32_t t0 = tmem_base + lane_addr + (uint32_t)((s * MT + m) * NT);
         // one 8-column sample group: wholly live or wholly dead, inside one centre; the centre's
         // first sample stands for its NS - ns pad copies as well (weight 1 + wx)
-        auto process = [&](const uint32_t (&r)[8], int sg) {
+        auto process = [&](uint32_t (&r)[8], int sg) {
           if (!c_ok) return;
           const int col0 = sg * 8;
           if (a.epilogue == 0) {   // dead rows are stored too: later layers must read finite z
-            float *zp = a.z + (size_t)(pos0 + col0) * a.Cout + c;
+            float *zp = a.z + (size_t)(pos0 + col0) * ldz + c;
+            if constexpr (SL) {
+              if (a.accumulate) {   // earlier feature slices' partial z first, then this product
 #pragma unroll
-            for (int i = 0; i < 8; ++i) zp[(size_t)i * a.Cout] = __uint_as_float(r[i]);
+                for (int i = 0; i < 8; ++i)
+                  r[i] = __float_as_uint(zp[(size_t)i * ldz] + __uint_as_float(r[i]));
+              }
+            }
+#pragma unroll
+            for (int i = 0; i < 8; ++i) zp[(size_t)i * ldz] = __uint_as_float(r[i]);
           }
           if (col0 >= tc.live) return;
           const int s0 = (p64 + col0) & nsm;
@@ -425,7 +443,7 @@ __global__ void __launch_bounds__(kFwdThreads, 1) sa_layer_fwd_kernel(const Laye
               if constexpr (CMP) centre = s_cene[(k & 1) * NT + col0];
               else centre = (pos0 + col0) >> a.ns_shift;
               if (centre >= 0) {
-                const size_t o = (size_t)centre * a.Cout + c;
+                const size_t o = (size_t)centre * ldz + c;
                 a.zmax[o] = mx; a.zmin[o] = mn; a.amax[o] = ax; a.amin[o] = an;
               }
             }
@@ -461,7 +479,7 @@ __global__ void __launch_bounds__(kFwdThreads, 1) sa_layer_fwd_kernel(const Laye
         const int c = m * 128 + q * 32 + lane;
         if (m < MT && c < a.Cout) {
           atomicAdd(a.stats + c, acc_s[m]);
-          atomicAdd(a.stats + a.Cout + c, acc_ss[m]);
+          atomicAdd(a.stats + ldz + c, acc_ss[m]);
         }
       }
     }
@@ -611,16 +629,63 @@ int fwd_pick_nt(int Kp, int Cout_pad, int Cin, int mode, int epilogue, int NS, l
   *raw_stage = 0;
   return 0;
 }
+
+// whether ONE launch can hold a layer of these channel counts at all: the narrowest tile (32
+// positions, register-staged) within shared memory and TMEM; compact: with a plan's extra words
+bool fwd_fits(int Cin, int Cout, int gather, int cmp) {
+  if (Cout > 256) return false;
+  const int Cout_pad = (Cout + 127) & ~127;
+  const FwdSmem L = fwd_smem_layout(packed_k(Cin, gather), Cout_pad, 32, 0, cmp);
+  return L.total <= 227u * 1024u && 2 * (Cout_pad >> 7) * 32 <= 512;
+}
 }  // namespace
+
+// Slice grid (include/b2r.h).  A layer that fits one launch keeps it.  Otherwise output slices of
+// 256 or 128 channels, and for gather layers (not pooled) feature slices of C/2, C/4, ... channels
+// (multiples of 8), checked with the plan's extra shared memory: the grid with the fewest launches,
+// then the fewest feature slices (each one after the first re-reads z).
+extern "C" int b2r_sa_layer_fwd_slices(int Cin, int Cout, int gather, int pooled, int *co_step,
+                                       int *ci_step) {
+  if (Cin <= 0 || Cout <= 0 || (gather && Cin < 3) || (!gather && (Cin % 4) != 0)) return 0;
+  int best = 0, best_kn = 0, bco = 0, bci = 0;
+  if (fwd_fits(Cin, Cout, gather, 0)) {
+    best = 1; bco = Cout; bci = 0;
+  } else if (Cout % 8 == 0) {
+    const int C = Cin - 3;
+    for (int cs : {256, 128}) {
+      const int co = cs < Cout ? cs : Cout;
+      for (int kn = 1; kn <= 16; kn *= 2) {
+        int ci = 0;
+        if (kn > 1) {
+          if (!gather || pooled || C % 8 != 0) break;
+          ci = ((C + kn - 1) / kn + 7) & ~7;
+          if (ci * (kn - 1) >= C) continue;
+        }
+        if (!fwd_fits(kn > 1 ? 3 + ci : Cin, co, gather, 1)) continue;
+        const int n = ((Cout + co - 1) / co) * (kn > 1 ? (C + ci - 1) / ci : 1);
+        if (best == 0 || n < best || (n == best && kn < best_kn)) {
+          best = n; best_kn = kn; bco = co; bci = ci;
+        }
+        break;   // more feature slices only add launches at this output width
+      }
+    }
+  }
+  if (co_step) *co_step = bco;
+  if (ci_step) *ci_step = bci;
+  return best;
+}
 
 extern "C" int b2r_sa_layer_fwd_supported(int B, int NP, int NS, int Cin, int Cout, int gather,
                                           int pooled) {
-  if (B <= 0 || NP <= 0 || NS <= 0 || Cin <= 0 || Cout <= 0 || Cout > 256) return 0;
+  if (B <= 0 || NP <= 0 || NS <= 0 || Cin <= 0 || Cout <= 0) return 0;
   if (gather ? Cin < 3 : (Cin % 4) != 0) return 0;
   if (pooled && !(NS == 16 || NS == 32 || NS == 64)) return 0;
+  int co = 0, ci = 0;
+  if (b2r_sa_layer_fwd_slices(Cin, Cout, gather, pooled, &co, &ci) == 0) return 0;
+  const int Cin_s = ci > 0 ? 3 + ci : Cin;   // the widest slice decides the tile
   const long long per_scene = (long long)NP * NS, M = (long long)B * per_scene;
   int raw = 0;
-  return fwd_pick_nt(packed_k(Cin, gather), (Cout + 127) & ~127, Cin, gather ? 0 : 1,
+  return fwd_pick_nt(packed_k(Cin_s, gather), (co + 127) & ~127, Cin_s, gather ? 0 : 1,
                      pooled ? 1 : 0, NS, M, per_scene, &raw) > 0 ? 1 : 0;
 }
 
@@ -641,17 +706,42 @@ extern "C" int b2r_sa_layer_fwd(const b2r_sa_layer *d, void *stream) {
   B2R_REQUIRE(d->mode == 0 || d->mode == 1, "b2r_sa_layer_fwd: mode must be 0 or 1");
   B2R_REQUIRE(d->epilogue == 0 || d->epilogue == 1, "b2r_sa_layer_fwd: epilogue must be 0 or 1");
   B2R_REQUIRE(d->w_image != nullptr, "b2r_sa_layer_fwd: null weight image");
+  const bool co_sliced = d->co_n != 0, ci_sliced = d->ci_n != 0;
+  B2R_REQUIRE(co_sliced ? (d->co0 >= 0 && d->co_n > 0 && d->co0 <= d->Cout - d->co_n)
+                        : d->co0 == 0,
+              "b2r_sa_layer_fwd: output slice [%d, +%d) outside Cout=%d", d->co0, d->co_n, d->Cout);
+  B2R_REQUIRE(!ci_sliced || (d->mode == 0 && d->epilogue == 0),
+              "b2r_sa_layer_fwd: feature slices are for gather layers that store z");
+  B2R_REQUIRE(ci_sliced ? (d->ci0 >= 0 && d->ci_n > 0 && d->ci0 <= d->Cin - 3 - d->ci_n &&
+                           d->ci0 % 8 == 0 && d->ci_n % 8 == 0)
+                        : d->ci0 == 0,
+              "b2r_sa_layer_fwd: feature slice [%d, +%d) outside the %d features or not a "
+              "multiple of 8", d->ci0, d->ci_n, d->Cin - 3);
+  B2R_REQUIRE(!d->accumulate || (d->accumulate == 1 && d->epilogue == 0),
+              "b2r_sa_layer_fwd: accumulate is 0, or 1 for a layer that stores z");
+  const int Cout_s = co_sliced ? d->co_n : d->Cout;
+  const int Cin_s = ci_sliced ? 3 + d->ci_n : d->Cin;
   LayerArgs a;
-  a.B = d->B; a.N = d->N; a.NP = d->NP; a.NS = d->NS; a.Cin = d->Cin; a.Cout = d->Cout;
+  // a slice launch: the kernel sees a layer of Cin_s -> Cout_s channels whose outputs sit at
+  // column co0 of the whole layer's rows and whose features start at column ci0 of feat_t's rows
+  const int co0 = d->co0;
+  a.B = d->B; a.N = d->N; a.NP = d->NP; a.NS = d->NS; a.Cin = Cin_s; a.Cout = Cout_s;
   a.mode = d->mode; a.epilogue = d->epilogue;
-  a.xyz = d->xyz; a.new_xyz = d->new_xyz; a.feat_t = d->feat_t; a.idx = d->idx;
+  a.xyz = d->xyz; a.new_xyz = d->new_xyz; a.idx = d->idx;
+  a.feat_t = d->feat_t != nullptr ? d->feat_t + d->ci0 : nullptr;
   a.radius = d->radius; a.normalize_xyz = d->normalize_xyz;
   a.z_prev = d->z_prev; a.scale_prev = d->scale_prev; a.shift_prev = d->shift_prev;
-  a.w_image = d->w_image; a.z = d->z; a.stats = d->stats;
-  a.zmax = d->zmax; a.zmin = d->zmin; a.amax = d->amax; a.amin = d->amin;
-  a.Kp = packed_k(d->Cin, d->mode == 0);
-  a.Cout_pad = (d->Cout + 127) & ~127;
-  a.chf_shift = pow2_shift(((d->Cin - 3 + 3) & ~3) >> 2);
+  a.w_image = d->w_image;
+  a.z = d->z != nullptr ? d->z + co0 : nullptr;
+  a.stats = d->stats != nullptr ? d->stats + co0 : nullptr;
+  a.zmax = d->zmax != nullptr ? d->zmax + co0 : nullptr;
+  a.zmin = d->zmin != nullptr ? d->zmin + co0 : nullptr;
+  a.amax = d->amax != nullptr ? d->amax + co0 : nullptr;
+  a.amin = d->amin != nullptr ? d->amin + co0 : nullptr;
+  a.ldz = d->Cout; a.ldf = d->Cin - 3; a.accumulate = d->accumulate;
+  a.Kp = packed_k(Cin_s, d->mode == 0);
+  a.Cout_pad = (Cout_s + 127) & ~127;
+  a.chf_shift = pow2_shift(((Cin_s - 3 + 3) & ~3) >> 2);
   a.ns_shift = pow2_shift(d->NS);
   a.cidx = d->cidx; a.ccen = d->ccen; a.cmeta = d->cmeta;
   const int cmp = d->cmeta != nullptr ? 1 : 0;
@@ -684,20 +774,22 @@ extern "C" int b2r_sa_layer_fwd(const b2r_sa_layer *d, void *stream) {
     }
   }
   if (a.Cout_pad > 256) {
-    set_error("b2r_sa_layer_fwd: needs Cout <= 256 (got %d)", d->Cout);
+    set_error("b2r_sa_layer_fwd: needs Cout <= 256 per launch (got %d; see "
+              "b2r_sa_layer_fwd_slices)", Cout_s);
     return B2R_ERR_UNSUPPORTED;
   }
   // thin first layer (Cin <= 8): a streaming CUDA-core kernel, not a tensor-core tile pipeline
-  if (thin::fwd_applicable(d)) return thin::fwd_launch(d, stream);
-  const int NT = fwd_pick_nt(a.Kp, a.Cout_pad, d->Cin, d->mode, d->epilogue, d->NS, M, per_scene,
+  if (!co_sliced && !ci_sliced && !d->accumulate && thin::fwd_applicable(d))
+    return thin::fwd_launch(d, stream);
+  const int NT = fwd_pick_nt(a.Kp, a.Cout_pad, Cin_s, d->mode, d->epilogue, d->NS, M, per_scene,
                              &a.raw_stage, cmp);
   if (NT == 0) {
     set_error("b2r_sa_layer_fwd: layer Cin=%d Cout=%d M=%lld NP*NS=%lld does not fit (needs "
               "B*NP*NS %% 32 == 0, gather layers NP*NS %% 32 == 0, operands within 227 KB)",
-              d->Cin, d->Cout, M, per_scene);
+              Cin_s, Cout_s, M, per_scene);
     return B2R_ERR_UNSUPPORTED;
   }
-  const FwdSmem L = fwd_smem_layout(a.Kp, a.Cout_pad, NT, a.raw_stage ? d->Cin : 0, cmp);
+  const FwdSmem L = fwd_smem_layout(a.Kp, a.Cout_pad, NT, a.raw_stage ? Cin_s : 0, cmp);
   a.num_tiles = (int)(M / NT);
   // persistent grid: one CTA per SM, or fewer when the caller keeps SMs free for kernels running
   // concurrently on another stream (the geometry pre-pass: FPS needs whole SMs to itself)
@@ -705,11 +797,16 @@ extern "C" int b2r_sa_layer_fwd(const b2r_sa_layer *d, void *stream) {
   if (d->sm_limit > 0 && d->sm_limit < kNumSMs) sms = d->sm_limit;
   const int grid = a.num_tiles < sms ? a.num_tiles : sms;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const bool sliced = co_sliced || ci_sliced || d->accumulate;
+#define B2R_LAUNCH_FWD2(NTV, CMPV, SLV)                                                         \
+  do {                                                                                          \
+    B2R_CUDA(cudaFuncSetAttribute(sa_layer_fwd_kernel<NTV, CMPV, SLV>,                          \
+                                  cudaFuncAttributeMaxDynamicSharedMemorySize, (int)L.total));  \
+    sa_layer_fwd_kernel<NTV, CMPV, SLV><<<grid, kFwdThreads, L.total, st>>>(a);                 \
+  } while (0)
 #define B2R_LAUNCH_FWD(NTV, CMPV)                                                               \
   do {                                                                                          \
-    B2R_CUDA(cudaFuncSetAttribute(sa_layer_fwd_kernel<NTV, CMPV>,                               \
-                                  cudaFuncAttributeMaxDynamicSharedMemorySize, (int)L.total));  \
-    sa_layer_fwd_kernel<NTV, CMPV><<<grid, kFwdThreads, L.total, st>>>(a);                      \
+    if (sliced) B2R_LAUNCH_FWD2(NTV, CMPV, true); else B2R_LAUNCH_FWD2(NTV, CMPV, false);       \
   } while (0)
   if (cmp) {
     if (NT == 128) B2R_LAUNCH_FWD(128, true);
@@ -721,6 +818,7 @@ extern "C" int b2r_sa_layer_fwd(const b2r_sa_layer *d, void *stream) {
     else B2R_LAUNCH_FWD(32, false);
   }
 #undef B2R_LAUNCH_FWD
+#undef B2R_LAUNCH_FWD2
   B2R_CHECK_LAUNCH();
   return B2R_OK;
 }

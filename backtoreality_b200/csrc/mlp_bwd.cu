@@ -35,6 +35,10 @@
 // then 1 MMA-issue warp (one thread), then the producers (global loads -> transform -> smem).  Two smem stages and two TMEM
 // stages for D1/D2, mbarrier hand-offs (full / empty / z_done / dz_ready / mma_done / d2_free):
 // producers run up to two tiles ahead of the tensor core, stores and scatters trail behind.
+// Layers beyond one launch's TMEM / shared memory run as channel-slice launches
+// (b2r_sa_layer_bwd_slices): an output slice adds its rows of dW and, dense layers, accumulates
+// its share of gr_prev after the first slice; a feature slice of a gather layer owns its dgrad
+// rows and dW columns.
 #include <cuda_bf16.h>
 
 #include "mlp_common.cuh"
@@ -71,6 +75,11 @@ struct BwdArgs {
   int ch8_shift;                         // log2(feature 16-byte chunks per row) or -1
   int ns_shift;                          // log2(NS) or -1
   const int *cidx, *ccen, *cmeta;        // compacted position space (csrc/compact.cu) or NULL
+  // channel slice (Cin / Cout above are the slice's): row pitch of dz / gr / z / dysel / asel (the
+  // whole layer's Cout), row pitch of feat_t / g_feat_t (the whole layer's features) and of dW
+  // (its Cin), first feature column of the slice in dW, whether the slice owns the xyz columns,
+  // and gr_prev += instead of gr_prev =
+  int ldo, ldf, ldw, kofs, xyz_cols, accumulate;
 };
 
 // packed K extent of a layer in THIS kernel's operand order: gather layers put the C feature
@@ -190,7 +199,9 @@ __global__ void pack_weight_bf16_kernel(const float *__restrict__ w, int Cout, i
 // dysel) and everything derived from them carry the positions' multiplicities implicitly: only
 // the DENSE BatchNorm-backward term b*z + c, which every padded position receives once, is
 // scaled by the multiplicity (1 + NS - class size for a centre's first sample, 0 for dead rows).
-template <int NT, int EW, int MODE, int TOP, bool CMP>
+// SL: a channel-slice launch (ldo / ldf / ldw / kofs / xyz_cols / accumulate); the whole-layer
+// instantiations keep the addressing they had before slices existed
+template <int NT, int EW, int MODE, int TOP, bool CMP, bool SL>
 __global__ void __launch_bounds__(kBwdThreads, 1) sa_layer_bwd_kernel(const BwdArgs a) {
   constexpr int kMode = MODE;
   constexpr bool kTop = TOP != 0;
@@ -232,6 +243,8 @@ __global__ void __launch_bounds__(kBwdThreads, 1) sa_layer_bwd_kernel(const BwdA
   constexpr uint32_t kTmemCols = 512;
   const long long per_scene = (long long)a.NP * a.NS;
   const int C = a.Cin - 3, Cf8 = (C + 7) & ~7;   // gather layers: feature channels
+  const int ldo = SL ? a.ldo : a.Cout;             // row pitch of dz / gr / z / dysel / asel
+  const int ldf = SL ? a.ldf : C;                  // row pitch of feat_t / g_feat_t
   int num_tiles = a.num_tiles;
   if constexpr (CMP) {
     num_tiles = __ldg(a.cmeta + 8) / NT;
@@ -300,10 +313,10 @@ __global__ void __launch_bounds__(kBwdThreads, 1) sa_layer_bwd_kernel(const BwdA
       if (ptid == 0 && tile + 2 * grid < num_tiles) {   // pull tile k+2 into L2 meanwhile
         const size_t pn = (size_t)(pos0 + 2ll * grid * NT);
         if (!kTop) {
-          if (!has_coef) prefetch_l2(a.dz + pn * a.Cout, (uint32_t)NT * a.Cout * 4u);
+          if (!has_coef) prefetch_l2(a.dz + pn * ldo, (uint32_t)NT * ldo * 4u);
           else {
-            prefetch_l2(a.gr + pn * a.Cout, (uint32_t)NT * a.Cout * 4u);
-            prefetch_l2(a.z + pn * a.Cout, (uint32_t)NT * a.Cout * 4u);
+            prefetch_l2(a.gr + pn * ldo, (uint32_t)NT * ldo * 4u);
+            prefetch_l2(a.z + pn * ldo, (uint32_t)NT * ldo * 4u);
           }
         }
         if (kMode == 1) prefetch_l2(a.z_prev + pn * a.Cin, (uint32_t)NT * a.Cin * 4u);
@@ -311,19 +324,28 @@ __global__ void __launch_bounds__(kBwdThreads, 1) sa_layer_bwd_kernel(const BwdA
       // ---- DZ tile from HBM (dense layers / direct dz); the top layer's DZ comes from D1 ------
       if (!kTop) {
         const int total = NT * CH8;
-        const size_t o0 = (size_t)pos0 * a.Cout;
+        const size_t o0 = (size_t)pos0 * ldo;
         for (int i0 = ptid; i0 < total; i0 += kProdThreads * 4) {
           float4 g[4][2], zz[4][2];
 #pragma unroll
           for (int u = 0; u < 4; ++u) {
             const int i = i0 + u * kProdThreads;
             if (i < total) {
+              // chunk i sits at float4 2 i of the tile for a whole layer, at row * ldo + ch * 8
+              // floats for a slice
+              size_t e = 0;
+              int e4 = 2 * i;
+              if constexpr (SL) {
+                const int row = ch8s >= 0 ? (i >> ch8s) : (i / CH8);
+                e = (size_t)row * ldo + (size_t)(i - row * CH8) * 8;
+                e4 = 0;
+              }
               if (!has_coef) {
-                const float4 *p = reinterpret_cast<const float4 *>(a.dz + o0) + 2 * i;
+                const float4 *p = reinterpret_cast<const float4 *>(a.dz + o0 + e) + e4;
                 g[u][0] = __ldg(p); g[u][1] = __ldg(p + 1);
               } else {
-                const float4 *p = reinterpret_cast<const float4 *>(a.gr + o0) + 2 * i;
-                const float4 *qz = reinterpret_cast<const float4 *>(a.z + o0) + 2 * i;
+                const float4 *p = reinterpret_cast<const float4 *>(a.gr + o0 + e) + e4;
+                const float4 *qz = reinterpret_cast<const float4 *>(a.z + o0 + e) + e4;
                 g[u][0] = __ldg(p); g[u][1] = __ldg(p + 1);
                 zz[u][0] = __ldg(qz); zz[u][1] = __ldg(qz + 1);
               }
@@ -414,7 +436,7 @@ __global__ void __launch_bounds__(kBwdThreads, 1) sa_layer_bwd_kernel(const BwdA
               make_uint4(pack_bf16(d0, d1), pack_bf16(d2, 0.f), 0u, 0u);
         }
         if (CH8f > 0) {
-          const float *fb = a.feat_t + (size_t)b * a.N * C;
+          const float *fb = a.feat_t + (size_t)b * a.N * ldf;
           const int total = NT * CH8f;
           if ((C & 7) == 0) {
             for (int i0 = ptid; i0 < total; i0 += kProdThreads * 4) {
@@ -426,7 +448,7 @@ __global__ void __launch_bounds__(kBwdThreads, 1) sa_layer_bwd_kernel(const BwdA
                   const int row = a.ch8_shift >= 0 ? (i >> a.ch8_shift) : (i / CH8f);
                   const int ch = i - row * CH8f;
                   const float4 *p =
-                      reinterpret_cast<const float4 *>(fb + (size_t)s_idx[row] * C) + 2 * ch;
+                      reinterpret_cast<const float4 *>(fb + (size_t)s_idx[row] * ldf) + 2 * ch;
                   t[u][0] = __ldg(p); t[u][1] = __ldg(p + 1);
                 }
               }
@@ -445,7 +467,7 @@ __global__ void __launch_bounds__(kBwdThreads, 1) sa_layer_bwd_kernel(const BwdA
           } else {
             for (int i = ptid; i < total; i += kProdThreads) {
               const int row = i / CH8f, ch = i - row * CH8f;
-              const float *src = fb + (size_t)s_idx[row] * C + ch * 8;
+              const float *src = fb + (size_t)s_idx[row] * ldf + ch * 8;
               float f[8];
 #pragma unroll
               for (int e = 0; e < 8; ++e) f[e] = (ch * 8 + e < C) ? __ldg(src + e) : 0.f;
@@ -603,7 +625,7 @@ __global__ void __launch_bounds__(kBwdThreads, 1) sa_layer_bwd_kernel(const BwdA
                   continue;
                 }
               }
-              const size_t o = (size_t)cg * a.Cout + co;
+              const size_t o = (size_t)cg * ldo + co;
               asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(
                                smem_u32(my_dy + c * a.Cout_pad + co)),
                            "l"(a.dysel + o)
@@ -745,12 +767,24 @@ __global__ void __launch_bounds__(kBwdThreads, 1) sa_layer_bwd_kernel(const BwdA
                 float zv[32];   // all 32 (L2-resident) loads in flight before the first store
 #pragma unroll
                 for (int i = 0; i < 32; ++i) zv[i] = __ldg(zp + (size_t)i * a.Cin);
+                if (SL && a.accumulate) {
+                  // a later output slice: add its share of dz W to the earlier slices' (the mask
+                  // and the sums below are linear in it, so partial sums add up)
 #pragma unroll
-                for (int i = 0; i < 32; ++i) {
-                  const float g = fmaf(zv[i], sc, sh) > 0.f ? __uint_as_float(r[i]) : 0.f;
-                  gp[(size_t)i * a.Cin] = g;
-                  t1 += g;
-                  t2 = fmaf(g, zv[i], t2);
+                  for (int i = 0; i < 32; ++i) {
+                    const float g = fmaf(zv[i], sc, sh) > 0.f ? __uint_as_float(r[i]) : 0.f;
+                    gp[(size_t)i * a.Cin] += g;
+                    t1 += g;
+                    t2 = fmaf(g, zv[i], t2);
+                  }
+                } else {
+#pragma unroll
+                  for (int i = 0; i < 32; ++i) {
+                    const float g = fmaf(zv[i], sc, sh) > 0.f ? __uint_as_float(r[i]) : 0.f;
+                    gp[(size_t)i * a.Cin] = g;
+                    t1 += g;
+                    t2 = fmaf(g, zv[i], t2);
+                  }
                 }
                 s1[m] += t1;
                 s2[m] += t2;
@@ -761,10 +795,10 @@ __global__ void __launch_bounds__(kBwdThreads, 1) sa_layer_bwd_kernel(const BwdA
               const int e = kp - Cf8;                 // 0..2 for the dx,dy,dz rows
               const bool is_xyz = (e >= 0 && e < 3);
               if (is_feat && a.g_feat_t != nullptr) {
-                float *gb = a.g_feat_t + (size_t)tile_b * a.N * C + kp;
+                float *gb = a.g_feat_t + (size_t)tile_b * a.N * ldf + kp;
 #pragma unroll
                 for (int i = 0; i < 32; ++i)
-                  atomicAdd(gb + (size_t)s_idx[cc * 32 + i] * C, __uint_as_float(r[i]));
+                  atomicAdd(gb + (size_t)s_idx[cc * 32 + i] * ldf, __uint_as_float(r[i]));
               } else if (is_xyz && (a.g_xyz != nullptr || a.g_new_xyz != nullptr)) {
                 float run = 0.f;
                 float *gx = a.g_xyz != nullptr ? a.g_xyz + (size_t)tile_b * a.N * 3 + e : nullptr;
@@ -839,15 +873,15 @@ __global__ void __launch_bounds__(kBwdThreads, 1) sa_layer_bwd_kernel(const BwdA
           const int kp = at * 32 + lane;   // this lane's packed input channel
           int kk = -1;
           if (kMode == 0) {
-            if (kp < C) kk = 3 + kp;
-            else if (kp >= Cf8 && kp < Cf8 + 3) kk = kp - Cf8;
+            if (kp < C) kk = 3 + (SL ? a.kofs : 0) + kp;
+            else if ((!SL || a.xyz_cols) && kp >= Cf8 && kp < Cf8 + 3) kk = kp - Cf8;
           } else if (kp < a.Cin) {
             kk = kp;
           }
           if (kk >= 0) {
             const int rows = min(32, a.Cout - co0);
             for (int rr = 0; rr < rows; ++rr)
-              atomicAdd(a.dW + (size_t)(co0 + rr) * a.Cin + kk, stg[rr * 33 + lane]);
+              atomicAdd(a.dW + (size_t)(co0 + rr) * (SL ? a.ldw : a.Cin) + kk, stg[rr * 33 + lane]);
           }
           __syncwarp();
         }
@@ -1003,17 +1037,66 @@ int bwd_pick_nt(const Geometry &g, int Cout, int mode, int top, int do_dgrad, in
   }
   return 0;
 }
+
+// whether ONE launch can hold a layer of these channel counts at all (dgrad on, the narrowest
+// tile, which also satisfies every nsample rule); compact: with a plan's extra shared memory
+bool bwd_fits(int Cin, int Cout, int gather, int top, int cmp) {
+  if (Cout > 256) return false;
+  const Geometry g = bwd_geometry(Cout, Cin, gather);
+  if (((g.KA + 1) >> 1) > 3) return false;
+  const int MTp = (g.KA + 1) >> 1, MTl = g.Cout_pad >> 7;
+  const BwdSmem L = bwd_smem_layout(g.Kp, g.KA, g.WA, Cout, g.Cout_pad, 32, top, cmp);
+  const int w12 = ((top && MTl > MTp) ? MTl : MTp) * 32;
+  return L.total <= 227u * 1024u && 2 * w12 + MTl * g.KA * 64 <= 512;
+}
 }  // namespace
+
+// Slice grid (include/b2r.h): the same search as b2r_sa_layer_fwd_slices over the backward's
+// limits (shared memory, TMEM columns, at most three 128-row dgrad tiles)
+extern "C" int b2r_sa_layer_bwd_slices(int Cin, int Cout, int gather, int top, int *co_step,
+                                       int *ci_step) {
+  int best = 0, best_kn = 0, bco = 0, bci = 0;
+  if (Cin > 0 && Cout > 0 && (Cout % 8) == 0 && (gather ? Cin >= 3 : (Cin % 8) == 0)) {
+    if (bwd_fits(Cin, Cout, gather, top, 0)) {
+      best = 1; bco = Cout; bci = 0;
+    } else {
+      const int C = Cin - 3;
+      for (int cs : {256, 128}) {
+        const int co = cs < Cout ? cs : Cout;
+        for (int kn = 1; kn <= 16; kn *= 2) {
+          int ci = 0;
+          if (kn > 1) {
+            if (!gather || top || C % 8 != 0) break;
+            ci = ((C + kn - 1) / kn + 7) & ~7;
+            if (ci * (kn - 1) >= C) continue;
+          }
+          if (!bwd_fits(kn > 1 ? 3 + ci : Cin, co, gather, top, 1)) continue;
+          const int n = ((Cout + co - 1) / co) * (kn > 1 ? (C + ci - 1) / ci : 1);
+          if (best == 0 || n < best || (n == best && kn < best_kn)) {
+            best = n; best_kn = kn; bco = co; bci = ci;
+          }
+          break;
+        }
+      }
+    }
+  }
+  if (co_step) *co_step = bco;
+  if (ci_step) *ci_step = bci;
+  return best;
+}
 
 extern "C" int b2r_sa_layer_bwd_supported(int B, int NP, int NS, int Cin, int Cout, int gather,
                                           int top) {
   if (B <= 0 || NP <= 0 || NS <= 0 || Cin <= 0 || Cout <= 0) return 0;
-  if (Cout > 256 || (Cout % 8) != 0 || (!gather && (Cin % 8) != 0) || (gather && Cin < 3)) return 0;
+  if ((Cout % 8) != 0 || (!gather && (Cin % 8) != 0) || (gather && Cin < 3)) return 0;
   if (top && pow2_shift(NS) < 0) return 0;
-  const Geometry g = bwd_geometry(Cout, Cin, gather);
+  int co = 0, ci = 0;
+  if (b2r_sa_layer_bwd_slices(Cin, Cout, gather, top, &co, &ci) == 0) return 0;
+  const int Cin_s = ci > 0 ? 3 + ci : Cin;   // the widest slice decides the tile
+  const Geometry g = bwd_geometry(co, Cin_s, gather);
   const long long per_scene = (long long)NP * NS, M = (long long)B * per_scene;
   // worst case for the tile choice: every gradient requested (dgrad on)
-  return bwd_pick_nt(g, Cout, gather ? 0 : 1, top, 1, NS, M, per_scene) > 0 ? 1 : 0;
+  return bwd_pick_nt(g, co, gather ? 0 : 1, top, 1, NS, M, per_scene) > 0 ? 1 : 0;
 }
 
 extern "C" int b2r_sa_layer_bwd_tile(int B, int NP, int NS, int Cin, int Cout, int gather, int top,
@@ -1049,25 +1132,52 @@ extern "C" int b2r_sa_layer_bwd(const b2r_sa_layer_bwd_desc *d, void *stream) {
               "b2r_sa_layer_bwd: non-positive size");
   B2R_REQUIRE(d->mode == 0 || d->mode == 1, "b2r_sa_layer_bwd: mode must be 0 or 1");
   B2R_REQUIRE(d->dW != nullptr, "b2r_sa_layer_bwd: null dW");
+  const bool co_sliced = d->co_n != 0, ci_sliced = d->ci_n != 0;
+  B2R_REQUIRE(co_sliced ? (d->co0 >= 0 && d->co_n > 0 && d->co0 <= d->Cout - d->co_n &&
+                           d->co0 % 8 == 0)
+                        : d->co0 == 0,
+              "b2r_sa_layer_bwd: output slice [%d, +%d) outside Cout=%d or not 8-aligned", d->co0,
+              d->co_n, d->Cout);
+  B2R_REQUIRE(!ci_sliced || d->mode == 0, "b2r_sa_layer_bwd: feature slices are for gather layers");
+  B2R_REQUIRE(ci_sliced ? (d->ci0 >= 0 && d->ci_n > 0 && d->ci0 <= d->Cin - 3 - d->ci_n &&
+                           d->ci0 % 8 == 0 && d->ci_n % 8 == 0)
+                        : d->ci0 == 0,
+              "b2r_sa_layer_bwd: feature slice [%d, +%d) outside the %d features or not a "
+              "multiple of 8", d->ci0, d->ci_n, d->Cin - 3);
+  B2R_REQUIRE(!d->accumulate || (d->accumulate == 1 && d->mode == 1),
+              "b2r_sa_layer_bwd: accumulate is 0, or 1 for a dense layer (gather layers always "
+              "scatter-add)");
+  const int Cout_s = co_sliced ? d->co_n : d->Cout;
+  const int Cin_s = ci_sliced ? 3 + d->ci_n : d->Cin;
+  const int co0 = d->co0;
   const bool top = d->dysel != nullptr;
   B2R_REQUIRE(d->dz != nullptr || (d->coef_a && d->coef_b && d->coef_c &&
                                    ((d->gr && d->z) || (top && d->asel))),
               "b2r_sa_layer_bwd: needs dz, or gr + z + coef_a/b/c, or dysel + asel + coef_a/b/c");
+  // a slice launch: the kernel sees a layer of Cin_s -> Cout_s channels; the pointers below are
+  // moved to the slice's first output channel / feature column, the pitches stay the layer's
+  auto off = [](const float *p, long long o) { return p != nullptr ? p + o : nullptr; };
   BwdArgs a;
-  a.B = d->B; a.N = d->N; a.NP = d->NP; a.NS = d->NS; a.Cin = d->Cin; a.Cout = d->Cout;
+  a.B = d->B; a.N = d->N; a.NP = d->NP; a.NS = d->NS; a.Cin = Cin_s; a.Cout = Cout_s;
   a.mode = d->mode;
   a.top = (d->dz == nullptr && top) ? 1 : 0;
-  a.xyz = d->xyz; a.new_xyz = d->new_xyz; a.feat_t = d->feat_t; a.idx = d->idx;
+  a.xyz = d->xyz; a.new_xyz = d->new_xyz; a.feat_t = off(d->feat_t, d->ci0); a.idx = d->idx;
   a.radius = d->radius; a.normalize_xyz = d->normalize_xyz;
   a.z_prev = d->z_prev; a.scale_prev = d->scale_prev; a.shift_prev = d->shift_prev;
   a.w_image = d->w_image_bf16;
-  a.dz = d->dz; a.gr = d->gr; a.z = d->z; a.dysel = d->dysel; a.asel = d->asel;
-  a.coef_a = d->coef_a; a.coef_b = d->coef_b; a.coef_c = d->coef_c;
-  a.dW = d->dW; a.gr_prev = d->gr_prev; a.stats_prev = d->stats_prev;
-  a.g_feat_t = d->g_feat_t; a.g_xyz = d->g_xyz; a.g_new_xyz = d->g_new_xyz;
-  const Geometry g = bwd_geometry(d->Cout, d->Cin, d->mode == 0);
+  a.dz = off(d->dz, co0); a.gr = off(d->gr, co0); a.z = off(d->z, co0);
+  a.dysel = off(d->dysel, co0); a.asel = d->asel != nullptr ? d->asel + co0 : nullptr;
+  a.coef_a = off(d->coef_a, co0); a.coef_b = off(d->coef_b, co0); a.coef_c = off(d->coef_c, co0);
+  a.dW = d->dW + (size_t)co0 * d->Cin; a.gr_prev = d->gr_prev; a.stats_prev = d->stats_prev;
+  a.g_feat_t = d->g_feat_t != nullptr ? d->g_feat_t + d->ci0 : nullptr;
+  // the xyz rows of a gather layer belong to the feature slice that starts at 0
+  a.g_xyz = d->ci0 == 0 ? d->g_xyz : nullptr;
+  a.g_new_xyz = d->ci0 == 0 ? d->g_new_xyz : nullptr;
+  a.ldo = d->Cout; a.ldf = d->Cin - 3; a.ldw = d->Cin; a.kofs = d->ci0;
+  a.xyz_cols = d->ci0 == 0 ? 1 : 0; a.accumulate = d->accumulate;
+  const Geometry g = bwd_geometry(Cout_s, Cin_s, d->mode == 0);
   a.Kp = g.Kp; a.KA = g.KA; a.WA = g.WA; a.Cout_pad = g.Cout_pad;
-  a.ch8_shift = pow2_shift((((d->Cin - 3 + 7) & ~7) >> 3));
+  a.ch8_shift = pow2_shift((((Cin_s - 3 + 7) & ~7) >> 3));
   a.ns_shift = pow2_shift(d->NS);
   a.cidx = d->cidx; a.ccen = d->ccen; a.cmeta = d->cmeta;
   const int cmp = d->cmeta != nullptr ? 1 : 0;
@@ -1084,8 +1194,8 @@ extern "C" int b2r_sa_layer_bwd(const b2r_sa_layer_bwd_desc *d, void *stream) {
   if (d->mode == 0) {
     B2R_REQUIRE(d->Cin >= 3 && d->xyz && d->new_xyz && (d->idx || cmp) && (d->feat_t || d->Cin == 3),
                 "b2r_sa_layer_bwd: gather mode needs xyz, new_xyz, idx (and feat_t when Cin > 3)");
-    a.do_dgrad = (d->g_feat_t != nullptr && d->Cin > 3) || d->g_xyz != nullptr ||
-                 d->g_new_xyz != nullptr;
+    a.do_dgrad = (a.g_feat_t != nullptr && Cin_s > 3) || a.g_xyz != nullptr ||
+                 a.g_new_xyz != nullptr;
   } else {
     B2R_REQUIRE(d->z_prev && d->scale_prev && d->shift_prev,
                 "b2r_sa_layer_bwd: dense mode needs z_prev/scale/shift");
@@ -1095,20 +1205,20 @@ extern "C" int b2r_sa_layer_bwd(const b2r_sa_layer_bwd_desc *d, void *stream) {
   B2R_REQUIRE(!(a.do_dgrad || a.top) || d->w_image_bf16 != nullptr,
               "b2r_sa_layer_bwd: null weight image");
   // thin first layer without an input gradient (SA1: xyz / height are leaves): streaming kernel
-  if (thin::bwd_applicable(d)) return thin::bwd_launch(d, stream);
+  if (!co_sliced && !ci_sliced && thin::bwd_applicable(d)) return thin::bwd_launch(d, stream);
   // with a plan the launch is sized for the plan's CAPACITY; the live tile count is on the device
   const long long M = cmp ? b2r_compact_capacity(d->B, d->NP, d->NS)
                           : (long long)d->B * d->NP * d->NS;
   const long long per_scene = (long long)d->NP * d->NS;
-  if (a.Cout_pad > 256 || (d->Cout % 8) != 0 || (d->mode == 1 && (d->Cin % 8) != 0)) {
-    set_error("b2r_sa_layer_bwd: needs Cout %% 8 == 0, Cout <= 256, dense Cin %% 8 == 0 "
-              "(Cin=%d Cout=%d)", d->Cin, d->Cout);
+  if (a.Cout_pad > 256 || (Cout_s % 8) != 0 || (d->mode == 1 && (d->Cin % 8) != 0)) {
+    set_error("b2r_sa_layer_bwd: needs Cout %% 8 == 0, Cout <= 256 per launch (see "
+              "b2r_sa_layer_bwd_slices), dense Cin %% 8 == 0 (Cin=%d Cout=%d)", Cin_s, Cout_s);
     return B2R_ERR_UNSUPPORTED;
   }
-  const int NT = bwd_pick_nt(g, d->Cout, d->mode, a.top, a.do_dgrad, d->NS, M, per_scene, cmp);
+  const int NT = bwd_pick_nt(g, Cout_s, d->mode, a.top, a.do_dgrad, d->NS, M, per_scene, cmp);
   if (NT == 0) {
     set_error("b2r_sa_layer_bwd: layer Cin=%d Cout=%d M=%lld does not fit shared memory / TMEM",
-              d->Cin, d->Cout, M);
+              Cin_s, Cout_s, M);
     return B2R_ERR_UNSUPPORTED;
   }
   const BwdSmem L = bwd_smem_layout(a.Kp, a.KA, a.WA, a.Cout, a.Cout_pad, NT, a.top, cmp);
@@ -1117,11 +1227,17 @@ extern "C" int b2r_sa_layer_bwd(const b2r_sa_layer_bwd_desc *d, void *stream) {
   if (d->sm_limit > 0 && d->sm_limit < kNumSMs) sms = d->sm_limit;
   const int grid = a.num_tiles < sms ? a.num_tiles : sms;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const bool sliced = co_sliced || ci_sliced || d->accumulate;
+#define B2R_LAUNCH_BWD3(NTV, EWV, MV, TV, CV, SLV)                                              \
+  do {                                                                                          \
+    B2R_CUDA(cudaFuncSetAttribute(sa_layer_bwd_kernel<NTV, EWV, MV, TV, CV, SLV>,               \
+                                  cudaFuncAttributeMaxDynamicSharedMemorySize, (int)L.total));  \
+    sa_layer_bwd_kernel<NTV, EWV, MV, TV, CV, SLV><<<grid, kBwdThreads, L.total, st>>>(a);      \
+  } while (0)
 #define B2R_LAUNCH_BWD2(NTV, EWV, MV, TV, CV)                                                   \
   do {                                                                                          \
-    B2R_CUDA(cudaFuncSetAttribute(sa_layer_bwd_kernel<NTV, EWV, MV, TV, CV>,                    \
-                                  cudaFuncAttributeMaxDynamicSharedMemorySize, (int)L.total));  \
-    sa_layer_bwd_kernel<NTV, EWV, MV, TV, CV><<<grid, kBwdThreads, L.total, st>>>(a);           \
+    if (sliced) B2R_LAUNCH_BWD3(NTV, EWV, MV, TV, CV, true);                                    \
+    else B2R_LAUNCH_BWD3(NTV, EWV, MV, TV, CV, false);                                          \
   } while (0)
 #define B2R_LAUNCH_BWD1(NTV, EWV, MV, TV)                                                       \
   do {                                                                                          \
@@ -1143,6 +1259,7 @@ extern "C" int b2r_sa_layer_bwd(const b2r_sa_layer_bwd_desc *d, void *stream) {
 #undef B2R_LAUNCH_BWD
 #undef B2R_LAUNCH_BWD1
 #undef B2R_LAUNCH_BWD2
+#undef B2R_LAUNCH_BWD3
   B2R_CHECK_LAUNCH();
   return B2R_OK;
 }

@@ -140,6 +140,7 @@ __host__ __device__ inline int packed_k(int Cin, int gather) {
 struct GatherSrc {
   const float *xyz, *new_xyz, *feat_t;
   int N, NP, NS, C, Cf4;
+  int ldf;         // row pitch of feat_t: C, or the whole layer's feature count for a slice
   int chf_shift;   // log2(Cf4/4) when that is a power of two, else -1
   float radius;
   int normalize_xyz;
@@ -170,7 +171,7 @@ __device__ __forceinline__ void build_x_gather(const GatherSrc &g, int b, int in
         make_uint4(to_tf32(d0), to_tf32(d1), to_tf32(d2), 0u);
   }
   if (CHf == 0) return;
-  const float *fb = g.feat_t + (size_t)b * g.N * C;
+  const float *fb = g.feat_t + (size_t)b * g.N * g.ldf;
   const int total = NT * CHf;
   if ((C & 3) == 0) {
     for (int i0 = tid; i0 < total; i0 += NTHREADS * 8) {
@@ -181,7 +182,7 @@ __device__ __forceinline__ void build_x_gather(const GatherSrc &g, int b, int in
         if (i < total) {
           const int row = g.chf_shift >= 0 ? (i >> g.chf_shift) : (i / CHf);
           const int ch = i - row * CHf;
-          t[u] = __ldg(reinterpret_cast<const float4 *>(fb + (size_t)s_idx[row] * C) + ch);
+          t[u] = __ldg(reinterpret_cast<const float4 *>(fb + (size_t)s_idx[row] * g.ldf) + ch);
         }
       }
 #pragma unroll
@@ -199,7 +200,7 @@ __device__ __forceinline__ void build_x_gather(const GatherSrc &g, int b, int in
     for (int i = tid; i < total; i += NTHREADS) {
       const int row = g.chf_shift >= 0 ? (i >> g.chf_shift) : (i / CHf);
       const int ch = i - row * CHf;
-      const float *src = fb + (size_t)s_idx[row] * C + ch * 4;
+      const float *src = fb + (size_t)s_idx[row] * g.ldf + ch * 4;
       float f[4] = {0.f, 0.f, 0.f, 0.f};
 #pragma unroll
       for (int e = 0; e < 4; ++e)

@@ -30,6 +30,7 @@ Pad-free position space (COMPACT, csrc/compact.cu): blocks with nsample >= 32 do
 copies of a ball's first hit that the ball query pads with; see `compact_plan`.
 """
 import ctypes
+import functools
 import os
 
 import torch
@@ -63,6 +64,53 @@ def pack_weight(weight, gather):
                                               _ext._stream()), "mlp_pack_weight")
     _ext.LAUNCHES += 1
     return image
+
+
+# ---- channel slices ----------------------------------------------------------------------------
+# A layer too large for one launch (GroupFree3D's width-2 backbone: 259/515 -> 256 gather layers,
+# 256 -> 256, 256 -> 512) runs as a fixed grid of launches, each over a slice of the output
+# channels and, for gather layers, of the feature channels.  The library chooses the grid
+# (b2r_sa_layer_fwd_slices / _bwd_slices); a layer that fits one launch gets the single entry
+# (0, 0, 0, 0), i.e. the whole-layer launch with every slice field zero.
+@functools.lru_cache(maxsize=None)
+def slice_grid(backward, Cin, Cout, gather, last):
+    """[(co0, co_n, ci0, ci_n)] in launch order: output slice by output slice, feature slices in
+    increasing order inside each."""
+    co, ci = ctypes.c_int(), ctypes.c_int()
+    fn = _lib.lib().b2r_sa_layer_bwd_slices if backward else _lib.lib().b2r_sa_layer_fwd_slices
+    n = fn(Cin, Cout, 1 if gather else 0, 1 if last else 0, ctypes.byref(co), ctypes.byref(ci))
+    if n <= 0:
+        raise RuntimeError("no fused launch grid for a %d -> %d layer" % (Cin, Cout))
+    if n == 1:
+        return ((0, 0, 0, 0),)
+    C = Cin - 3
+    fs = [(c0, min(ci.value, C - c0)) for c0 in range(0, C, ci.value)] if ci.value else [(0, 0)]
+    grid = tuple((o0, min(co.value, Cout - o0), c0, cn)
+                 for o0 in range(0, Cout, co.value) for c0, cn in fs)
+    assert len(grid) == n, (grid, n)
+    return grid
+
+
+def _slice_weight(w, co0, co_n, ci0, ci_n):
+    """Weight (Cout,Cin) of one slice: rows co0.., and for a feature slice the columns
+    [xyz, features ci0..ci0+ci_n) with the xyz columns zero unless ci0 == 0 (they enter once)."""
+    if co_n == 0:
+        return w
+    w = w[co0:co0 + co_n]
+    if ci_n:
+        xyz = w[:, :3] if ci0 == 0 else torch.zeros_like(w[:, :3])
+        w = torch.cat([xyz, w[:, 3 + ci0:3 + ci0 + ci_n]], 1)
+    return w.contiguous()
+
+
+def pack_layer(weight, gather, kind, last):
+    """One operand image per launch of the layer's slice grid: "tf32" (forward) or "bf16"
+    (backward)."""
+    Cout, Cin = weight.shape[0], weight.shape[1]
+    w = weight.detach().reshape(Cout, Cin)
+    pack = pack_weight if kind == "tf32" else pack_weight_bf16
+    return [pack(_slice_weight(w, *sl), gather)
+            for sl in slice_grid(kind == "bf16", Cin, Cout, gather, last)]
 
 
 # ---- weight images packed ahead of time, off the critical path -------------------------------
@@ -110,8 +158,10 @@ def prepack(mlp_modules, backward=None):
                     w = blk.conv.weight
                     if kind == "bf16" and not w.requires_grad:
                         continue
-                    image = (pack_weight if kind == "tf32" else pack_weight_bf16)(w, gather=(i == 0))
-                    entries.append(((id(w), kind), image, w._version, w))
+                    images = pack_layer(w, i == 0, kind, i == len(mlp) - 1)
+                    # a one-launch layer keeps its single image, a sliced one the list
+                    entries.append(((id(w), kind), images[0] if len(images) == 1 else images,
+                                    w._version, w))
                 ev = torch.cuda.Event()
                 ev.record(side)
                 _PACK_EVENTS[dev].append(ev)
@@ -138,8 +188,14 @@ def _take(weight, kind):
     image, ev = ent[0], ent[1]
     main = torch.cuda.current_stream(weight.device)
     main.wait_event(ev)
-    image.record_stream(main)
+    for im in _as_list(image):
+        im.record_stream(main)
     return image
+
+
+def _as_list(image):
+    """A `_take` result as the list of per-slice images (one entry for a one-launch layer)."""
+    return [image] if torch.is_tensor(image) else image
 
 
 # Pad-free position space (csrc/compact.cu): the ball query pads a centre's unused slots with
@@ -194,6 +250,7 @@ def supported(mlp_module, xyz, features, idx, pooling="max"):
             return False
         cout, cin = blk.conv.out_channels, blk.conv.in_channels
         gather, top = (1 if i == 0 else 0), (1 if i == len(blocks) - 1 else 0)
+        # (both answer for the layer's slice grid when it does not fit one launch)
         if not lib.b2r_sa_layer_fwd_supported(B, NP, NS, cin, cout, gather, top):
             return False
         if not lib.b2r_sa_layer_bwd_supported(B, NP, NS, cin, cout, gather, top):
@@ -252,8 +309,7 @@ def sa_mlp_forward(xyz, new_xyz, feat_t, idx, radius, normalize_xyz, mlp_module,
         Cin, Cout = conv.in_channels, conv.out_channels
         last = i == L - 1
         image = _take(conv.weight, "tf32")
-        if image is None:
-            image = pack_weight(conv.weight, gather=(i == 0))
+        image = pack_layer(conv.weight, i == 0, "tf32", last) if image is None else _as_list(image)
         images.append(image)
         stats = None
         if training:
@@ -268,7 +324,6 @@ def sa_mlp_forward(xyz, new_xyz, feat_t, idx, radius, normalize_xyz, mlp_module,
             d.radius, d.normalize_xyz = float(radius), 1 if normalize_xyz else 0
         else:
             d.z_prev, d.scale_prev, d.shift_prev = _ptr(z_prev), _ptr(scale), _ptr(shift)
-        d.w_image = _ptr(image)
         d.sm_limit = int(sm_limit)
         if plan is not None:
             d.cidx, d.ccen, d.cmeta = _ptr(plan["cidx"]), _ptr(plan["ccen"]), _ptr(plan["cmeta"])
@@ -282,9 +337,17 @@ def sa_mlp_forward(xyz, new_xyz, feat_t, idx, radius, normalize_xyz, mlp_module,
         else:
             z = torch.empty((rows, Cout), dtype=torch.float32, device=dev)
             d.z = _ptr(z)
-        d.stats = _ptr(stats)
+        grid = slice_grid(False, Cin, Cout, i == 0, last)
         with _ext._timed("sa_layer_fwd", _layer_work(B, N, NP, NS, Cin, Cout, i == 0, last, False)):
-            _lib.check(lib.b2r_sa_layer_fwd(ctypes.byref(d), st), "sa_layer_fwd")
+            for (co0, co_n, ci0, ci_n), img in zip(grid, image):
+                # feature slices of one output slice: the first writes z, the others add to it,
+                # and the last one takes the BatchNorm sums of the finished z
+                d.co0, d.co_n, d.ci0, d.ci_n = co0, co_n, ci0, ci_n
+                d.accumulate = 1 if ci0 > 0 else 0
+                d.stats = _ptr(stats) if ci0 + ci_n >= Cin - 3 or ci_n == 0 else None
+                d.w_image = _ptr(img)
+                _lib.check(lib.b2r_sa_layer_fwd(ctypes.byref(d), st), "sa_layer_fwd")
+            _ext.LAUNCHES += len(grid) - 1   # (_timed counts one)
         # BatchNorm scale / shift of THIS layer (applied by the next layer's prologue / finalize)
         if training:
             scale = torch.empty(Cout, dtype=torch.float32, device=dev)
@@ -415,14 +478,21 @@ def sa_mlp_backward(g_out_cm, xyz, new_xyz, feat_t, idx, radius, normalize_xyz, 
             gr_prev = torch.empty((rows, Cin), **f32)
             stats_prev = stats_all[s_off[l - 1]:s_off[l]]
             b.gr_prev, b.stats_prev = _ptr(gr_prev), _ptr(stats_prev)
-        image = None
+        grid = slice_grid(True, Cin, Cout, l == 0, l == top)
+        images = [None] * len(grid)
         if need_dgrad or l == top:
-            image = _take(versioned[l], "bf16") if versioned is not None else None
-            if image is None:
-                image = pack_weight_bf16(weights[l], gather=(l == 0))
-        b.w_image_bf16 = _ptr(image)
+            images = _take(versioned[l], "bf16") if versioned is not None else None
+            images = (pack_layer(weights[l], l == 0, "bf16", l == top) if images is None
+                      else _as_list(images))
         with _ext._timed("sa_layer_bwd", _layer_work(B, N, NP, NS, Cin, Cout, l == 0, l == top, True)):
-            _lib.check(lib.b2r_sa_layer_bwd(ctypes.byref(b), st), "sa_layer_bwd")
+            for j, ((co0, co_n, ci0, ci_n), img) in enumerate(zip(grid, images)):
+                # dense layers: every output slice after the first adds its share of the input
+                # gradient (launch order fixes the summation order); gather layers scatter-add
+                b.co0, b.co_n, b.ci0, b.ci_n = co0, co_n, ci0, ci_n
+                b.accumulate = 1 if (l > 0 and j > 0) else 0
+                b.w_image_bf16 = _ptr(img)
+                _lib.check(lib.b2r_sa_layer_bwd(ctypes.byref(b), st), "sa_layer_bwd")
+            _ext.LAUNCHES += len(grid) - 1
         if l > 0:
             mean, invstd, _, _ = bn[l - 1]
             coef = [torch.empty(Cin, **f32) for _ in range(3)]

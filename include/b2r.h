@@ -226,8 +226,9 @@ B2R_API int b2r_query_group_bwd(const float *grad_out, const int *idx, int B, in
  *               b2r_pool_finalize turns them into max_pool(relu(bn(z))) exactly
  * Weights are passed as the packed image produced by b2r_mlp_pack_weight (TF32-rounded,
  * 128-byte-swizzled K-major shared-memory layout, staged by one TMA bulk copy).
- * Limits: Cout <= 256, B*NP*NS % 32 == 0 (gather layers: NP*NS % 32 == 0), NS in {16,32,64}
- * for epilogue 1; otherwise B2R_ERR_UNSUPPORTED (callers then use the unfused path).
+ * Limits: Cout <= 256 per launch (wider layers: the channel slices below), B*NP*NS % 32 == 0
+ * (gather layers: NP*NS % 32 == 0), NS in {16,32,64} for epilogue 1; otherwise
+ * B2R_ERR_UNSUPPORTED (callers then use the unfused path).
  */
 typedef struct b2r_sa_layer {
   int B, N, NP, NS;   /* scenes, source points per scene, centres per scene, samples per centre */
@@ -256,6 +257,17 @@ typedef struct b2r_sa_layer {
    * and the number of tiles is read from cmeta on the device.  amax / amin are then sample
    * indices inside the centre's class-size run (consistent with b2r_sa_layer_bwd). */
   const int *cidx, *ccen, *cmeta;
+  /* Channel slice (all zero = the whole layer in one launch).  A layer too large for one launch
+   * runs as the grid of launches b2r_sa_layer_fwd_slices gives; each launch covers output channels
+   * [co0, co0 + co_n) (co_n = 0: all) and, for gather layers, feature channels [ci0, ci0 + ci_n)
+   * (ci_n = 0: all; ci0 and ci_n multiples of 8).  Cin / Cout stay the WHOLE layer's; z, stats,
+   * zmax/zmin/amax/amin keep the whole layer's pitch and the launch writes its own columns.
+   * w_image packs the slice's weight: rows co0.., columns [xyz, features ci0..ci0+ci_n), with the
+   * xyz columns ZERO unless ci0 == 0 (b2r_mlp_pack_weight(w_slice, co_n, 3 + ci_n, 1, ...)).
+   * accumulate != 0 (epilogue 0 only): z += this launch's partial product instead of z = ...; the
+   * feature slices of one output slice run in increasing ci0 order, the first with accumulate = 0,
+   * and only the last passes stats (they are sums over the finished z). */
+  int co0, co_n, ci0, ci_n, accumulate;
 } b2r_sa_layer;
 
 B2R_API long long b2r_mlp_weight_image_bytes(int Cout, int Cin, int gather);
@@ -263,9 +275,18 @@ B2R_API long long b2r_mlp_weight_image_bytes(int Cout, int Cin, int gather);
 B2R_API int b2r_mlp_pack_weight(const float *w, int Cout, int Cin, int gather, float *image,
                                 void *stream);
 B2R_API int b2r_sa_layer_fwd(const b2r_sa_layer *desc, void *stream);
-/* 1 when b2r_sa_layer_fwd covers a layer of this shape, 0 otherwise (same rules as the launch). */
+/* 1 when b2r_sa_layer_fwd covers a layer of this shape, in one launch or in the channel slices of
+ * b2r_sa_layer_fwd_slices, 0 otherwise (same rules as the launch). */
 B2R_API int b2r_sa_layer_fwd_supported(int B, int NP, int NS, int Cin, int Cout, int gather,
                                        int pooled);
+
+/* Slice grid of a layer (depends on the channel counts only): returns the number of launches
+ * (0 = not covered; 1 = the whole layer, *co_step = Cout and *ci_step = 0).  Output slices are
+ * [j*co_step, min(Cout, (j+1)*co_step)); gather layers may also be cut into feature slices
+ * [i*ci_step, min(Cin-3, (i+1)*ci_step)) (ci_step = 0: none).  Launch order: output slice by
+ * output slice, feature slices in increasing order inside each. */
+B2R_API int b2r_sa_layer_fwd_slices(int Cin, int Cout, int gather, int pooled, int *co_step,
+                                    int *ci_step);
 
 /* Positions per tile the launch would use for a layer of this shape (0 = unsupported); compact:
  * with a b2r_compact_plan.  Diagnostic (DESIGN.md tile table, tests). */
@@ -346,6 +367,17 @@ typedef struct b2r_sa_layer_bwd_desc {
   const int *cidx, *ccen, *cmeta; /* as b2r_sa_layer: the forward's plan (gr, z, z_prev, gr_prev
                                are then in its position space; gradients carry the positions'
                                multiplicities, see csrc/compact.cu) */
+  /* Channel slice, as b2r_sa_layer (all zero = the whole layer; grid from
+   * b2r_sa_layer_bwd_slices).  dz / gr / z / dysel / asel keep the whole layer's pitch (Cout) and
+   * coef_a/b/c the whole layer's length; the launch reads its output channels [co0, co0 + co_n)
+   * and adds rows co0.. (and, gather layers, the columns of its feature slice) of dW.  A feature
+   * slice computes the gradient of its own feature channels; the xyz / centre gradients belong to
+   * the slice with ci0 == 0 (g_xyz, g_new_xyz are ignored by the others).
+   * accumulate != 0 (dense layers only): gr_prev += this slice's (dz W) * mask instead of
+   * gr_prev = ...; every output slice after the first passes it, and all add their partial
+   * BatchNorm-backward sums into stats_prev.  Gather layers always scatter-add, so the flag is
+   * rejected there (B2R_ERR_INVALID_ARG). */
+  int co0, co_n, ci0, ci_n, accumulate;
 } b2r_sa_layer_bwd_desc;
 
 B2R_API long long b2r_mlp_weight_bf16_image_bytes(int Cout, int Cin, int gather);
@@ -356,6 +388,9 @@ B2R_API int b2r_sa_layer_bwd(const b2r_sa_layer_bwd_desc *desc, void *stream);
  * 0 otherwise: lets the host decide BEFORE the forward whether to take the fused path. */
 B2R_API int b2r_sa_layer_bwd_supported(int B, int NP, int NS, int Cin, int Cout, int gather,
                                        int top);
+/* Slice grid of the backward, as b2r_sa_layer_fwd_slices (sized for dgrad on). */
+B2R_API int b2r_sa_layer_bwd_slices(int Cin, int Cout, int gather, int top, int *co_step,
+                                    int *ci_step);
 
 B2R_API int b2r_sa_layer_bwd_tile(int B, int NP, int NS, int Cin, int Cout, int gather, int top,
                                   int dgrad, int compact);
